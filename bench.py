@@ -20,6 +20,9 @@ A "step" is one scheduling cycle of the hot path over every pool this process ow
            includes ranking, rebalancing and the exchange - not only the matcher.
   e2e    : the same step through the C ABI with HOST buffers, H2D + D2H inside, wall clock.
   --impl reference : the reference algorithm's CPU restatement on the host cores, same step.
+  --dump-outputs DIR : after the timed steps, what the last resident step returned to its caller
+           (rank, match, rebalance results per pool and the gathered usage) as DIR/<name>.npy,
+           float64, at most 64 MB in all; inputs are seeded, so two builds compare file by file.
 """
 import argparse
 import json
@@ -28,9 +31,11 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 import numpy as np
 
+sys.dont_write_bytecode = True   # the benchmark may run from a read-only tree: no caches written into it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -257,14 +262,16 @@ def run_ours(args):
     has_reb = cfg in ("c4", "c5")
 
     def cycle(resident):
-        """One scheduling cycle over this rank's pools.  Returns per-phase device ms, evals, placements."""
+        """One scheduling cycle over this rank's pools.  Returns per-phase device ms, evals, placements,
+        and what the calls returned: {pool: (rank, match, rebalance)} and the gathered usage."""
         ph = {"rank": 0.0, "match": 0.0, "match_kernel": 0.0, "rebalance": 0.0, "exchange": 0.0}
         ev = pl = ln = h2d = d2h = dec = 0
         last = None
+        outs = {}
         for i in range(slots):
             pr = pools[i] if i < len(pools) else None
             if pr is not None:
-                pr.rank()
+                r = pr.rank()
                 s = pr.eng.last_stats(abi.PHASE_RANK)
                 ph["rank"] += s["ms_device"]; ln += s["n_launches"]; h2d += s["h2d_bytes"]; d2h += s["d2h_bytes"]
                 m = pr.match(resident)
@@ -272,11 +279,13 @@ def run_ours(args):
                 ph["match"] += s["ms_considerable"] + s["ms_match"]; ph["match_kernel"] += s["ms_match_kernel"]
                 ev += s["evals"]; pl += s["n_matched"]; ln += s["n_launches"]; h2d += s["h2d_bytes"]; d2h += s["d2h_bytes"]
                 last = s
+                d = None
                 if has_reb:
                     d = pr.rebalance()
                     dec += len(d)
                     s = pr.eng.last_stats(abi.PHASE_REBALANCE)
                     ph["rebalance"] += s["ms_device"]; h2d += s["h2d_bytes"]; d2h += s["d2h_bytes"]
+                outs[pr.p] = (r, m, d)
         # ONE exchange per cycle for all of this rank's pools (cook_exchange_usage_batch): LPT balances the
         # SUM of a rank's pools; a collective per pool slot would make every slot as long as its slowest rank
         g = exchange_usage_batch([q.eng for q in pools], nu_pad, n_slots=slots, comm=comm, world=world)   # [world, slots, nu_pad, 4]
@@ -287,7 +296,7 @@ def run_ours(args):
         tot = g.sum(axis=(0, 1, 2))
         for q in pools:
             q.group_usage = tot
-        return ph, ev, pl, ln, h2d, d2h, dec, last
+        return ph, ev, pl, ln, h2d, d2h, dec, last, (outs, g)
 
     # ---------------- resident-input arm (value): upload once, then reuse_resident
     cycle(False)
@@ -306,7 +315,7 @@ def run_ours(args):
     for _ in range(args.steps):
         flush.zero_()  # L2 flush between timed iterations (outside the device-timed region)
         torch.cuda.synchronize()
-        ph, ev, pl, ln, _, _, dec, last = cycle(True)
+        ph, ev, pl, ln, _, _, dec, last, outputs = cycle(True)
         for k in tot:
             tot[k] += ph[k]
         evals += ev; places += pl; launches += ln; decisions += dec
@@ -327,7 +336,7 @@ def run_ours(args):
     h2d = d2h = 0
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        _, _, _, _, h2d, d2h, _, _ = cycle(False)
+        _, _, _, _, h2d, d2h, _, _, _ = cycle(False)
     barrier()
     e2e_s = max_over_ranks(time.perf_counter() - t0)
     h2d_all, d2h_all = sum_over_ranks(h2d), sum_over_ranks(d2h)
@@ -440,12 +449,58 @@ def run_ours(args):
         if cpu:
             line["cpu_baseline"] = cpu
         emit(line)
+    if args.dump_outputs:
+        outs, gathered = outputs
+        # every rank writes its own pools; the gathered usage is the same on all ranks
+        dump_outputs(args.dump_outputs, output_arrays(outs, gathered if rank == 0 else None), DUMP_BYTES // world)
     for pr in pools:
         pr.eng.close()
     if comm is not None:
         lib.cook_comm_destroy(comm)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64_000_000   # --dump-outputs: all files of all ranks together
+
+
+def output_arrays(outs, gathered=None):
+    """What a caller of the cycle receives, by name, in float64 (exact for the integer columns).
+    outs: {pool: (rank result, match result, rebalance decisions or None)}; gathered: the exchange's
+    [world, slots, users, 4] usage table, stored as rows of 4 (count, cpus, mem, gpus)."""
+    arrays = {}
+    for p, (r, m, d) in sorted(outs.items()):
+        for k in ("ranked", "dru", "order"):
+            arrays[f"pool{p:02d}_rank_{k}"] = r[k]
+        for k in ("considerable", "assign", "ports", "fail"):
+            arrays[f"pool{p:02d}_match_{k}"] = m[k]
+        if d is not None:
+            # one row per decision: pending_idx, host, number of victims, dru, mem, cpus, gpus
+            arrays[f"pool{p:02d}_rebalance_decisions"] = np.array(
+                [(x["pending_idx"], x["host"], len(x["victims"]), x["dru"], x["mem"], x["cpus"], x["gpus"]) for x in d],
+                np.float64).reshape(-1, 7)
+            arrays[f"pool{p:02d}_rebalance_victims"] = np.array([v for x in d for v in x["victims"]], np.float64)
+    if gathered is not None:
+        arrays["exchange_usage"] = gathered.reshape(-1, 4)
+    return {k: np.asarray(v, np.float64) for k, v in arrays.items()}
+
+
+def dump_outputs(out_dir, arrays, budget_bytes):
+    """Writes every array as out_dir/<name>.npy within budget_bytes.  When they do not fit, each array
+    keeps the same share of its rows, drawn by a generator seeded with the array's name (the same rows
+    in every run), and the numbers of the kept rows go to out_dir/<name>.rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    room = (budget_bytes - 512 * len(arrays)) // 8      # float64 values; 512 B per array for headers and rounding
+    total = sum(a.size for a in arrays.values())
+    share = 1.0 if total <= room else room / sum(a.size + a.shape[0] for a in arrays.values())
+    for name, a in arrays.items():
+        if share < 1.0 and a.shape[0] > 1:
+            rows = np.random.default_rng(zlib.crc32(name.encode())).choice(
+                a.shape[0], max(1, int(a.shape[0] * share)), replace=False)
+            rows.sort()
+            np.save(os.path.join(out_dir, name + ".rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_reference(args):
@@ -548,7 +603,12 @@ def main():
     ap.add_argument("--config", default="c2", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-nonsat", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -76,6 +76,40 @@ def test_nonsaturating_c2_variant_places_everything(oracle):
     assert m["stats"]["n_matched"] == 4000
 
 
+def test_dump_outputs_fits_its_budget_and_samples_the_same_rows(oracle, tmp_path):
+    """bench.py --dump-outputs: float64 files of the cycle's results; over budget, a fixed sample of
+    rows whose numbers are stored beside it, the same in every run."""
+    import bench
+    t = traces.gen_config_pool("c4", 3, scale=0.01)
+    r = oracle.rank(t["running"], t["pending"], t["users"])
+    m = oracle.match(r["ranked"], t["jobs"], t["offers"], t["users"],
+                     traces.match_params(t["jobs"].n, host_lifetime_mins=t["host_lifetime_mins"]),
+                     groups=t["groups"], max_ports=2)
+    rb = t["rebalance"]
+    d = oracle.rebalance(rb["running"], rb["pending"], rb["pending_job_id"], rb["pending_priority"], rb["hosts"],
+                         rb["users"], rb["params"], groups=rb["groups"])
+    assert len(d) > 0
+    arrays = bench.output_arrays({3: (r, m, d)}, np.arange(2 * 8 * 4.0).reshape(1, 2, 8, 4))
+    assert all(a.dtype == np.float64 for a in arrays.values())
+    assert np.array_equal(arrays["pool03_match_assign"], m["assign"])
+    assert arrays["pool03_rebalance_decisions"].shape == (len(d), 7)
+    assert arrays["exchange_usage"].shape == (16, 4)
+    full = sum(a.nbytes for a in arrays.values())
+    bench.dump_outputs(str(tmp_path / "all"), arrays, 2 * full)
+    for k, a in arrays.items():
+        assert np.array_equal(np.load(tmp_path / "all" / (k + ".npy")), a, equal_nan=True), k
+    budget = full // 4
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays, budget)
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= budget
+    for k, a in arrays.items():
+        got = np.load(tmp_path / "a" / (k + ".npy"))
+        assert got.dtype == np.float64 and np.array_equal(got, np.load(tmp_path / "b" / (k + ".npy")), equal_nan=True)
+        if len(a) > 1:
+            rows = np.load(tmp_path / "a" / (k + ".rows.npy")).astype(np.int64)
+            assert 0 < len(rows) < len(a) and np.array_equal(got, a[rows], equal_nan=True), k
+
+
 def test_reference_arm_prints_one_json_line():
     """The driver's contract: `bench.py --impl reference` runs on the host cores alone and prints exactly ONE
     line on stdout - the JSON with the arm's own cpu_baseline and e2e blocks (everything else, including what

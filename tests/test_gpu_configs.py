@@ -300,6 +300,31 @@ def test_placement_failure_summaries(gpu, oracle):
     assert len(seen & set(CONSTRAINT_NAMES)) >= 3   # several kinds of constraint failure occur in the trace
 
 
+def test_bench_dumps_what_its_last_timed_step_computed(oracle, tmp_path):
+    """bench.py --steps 2 --dump-outputs on C2: one JSON line reporting the 2 timed steps, and the dumped
+    queue, considerable set and assignments are the oracle's on the same seeded inputs."""
+    import json
+    import subprocess
+    import sys
+    import bench
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    p = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "1",
+                        "--no-cpu-baseline", "--no-nonsat", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=900, cwd=root)
+    assert p.returncode == 0, p.stderr[-2000:]
+    lines = p.stdout.splitlines()
+    assert len(lines) == 1 and json.loads(lines[0])["steps"] == 2
+    t = bench.gen_pool_inputs("c2", 0)
+    ro = oracle.rank(t["running"], t["pending"], t["users"])
+    mo = oracle.match(ro["ranked"], t["jobs"], t["offers"], t["users"], traces.match_params(t["jobs"].n),
+                      threads=min(64, os.cpu_count() or 1))
+    for name, want in (("rank_ranked", ro["ranked"]), ("rank_dru", ro["dru"]), ("match_considerable", mo["considerable"]),
+                       ("match_assign", mo["assign"])):
+        got = np.load(tmp_path / f"pool00_{name}.npy")
+        assert got.dtype == np.float64 and np.array_equal(got, want, equal_nan=True), name
+    assert np.load(tmp_path / "exchange_usage.npy")[:, 0].sum() == mo["stats"]["n_matched"] > 0
+
+
 def test_bad_index_columns_are_rejected_not_faulted(gpu):
     """A bad index from the shim comes back as COOK_E_BADARG (-1); the context stays usable."""
     from cook_b200.engine import CookError
