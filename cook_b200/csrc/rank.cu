@@ -56,13 +56,20 @@ struct LessUserTask {
 // with the smallest (dru, -arrival, name) where arrival = step at which the
 // user's previous task was emitted (0 for a user's first task): the popped
 // user's remainder is consed to the FRONT before a STABLE re-sort (:93-94).
-// Hence for equal dru:  X before Y  <=>  prev(X) was emitted AFTER prev(Y),
-// which recurses on the previous tasks with the roles swapped.
+// A popped user whose next task has the same dru is therefore popped again: a
+// user's RUN of equal-dru tasks (run_start) is emitted as one block, and the
+// blocks of one dru value go in the order their heads held when the first of
+// them came up.  Hence for equal dru:  X before Y  <=>  the task before X's run
+// was emitted AFTER the task before Y's run, which recurses on those two tasks
+// (smaller dru) with the roles swapped.  (Comparing prev(X) with prev(Y) instead
+// is only right for runs of one task: with a longer run, X's whole run goes out
+// before a later-arriving Y even becomes a head.)
 struct LessMerge {
   const double* dru;        // by sorted position; NaN = cut by limit-over-quota
   const int32_t* user_at;   // user of sorted position
   const int32_t* seg_start; // per user
   const int32_t* name_rank;
+  const int32_t* run_start; // by sorted position: first position of its user's run of equal dru
   __device__ bool operator()(int32_t x, int32_t y) const {
     double dx = dru[x], dy = dru[y];
     bool kx = dx == dx, ky = dy == dy;
@@ -72,17 +79,52 @@ struct LessMerge {
       if (dx != dy) return dx < dy;
       int ux = user_at[x], uy = user_at[y];
       if (ux == uy) return x < y;  // same user: queue order
-      bool hx = x > seg_start[ux], hy = y > seg_start[uy];
+      const int rx = run_start[x], ry = run_start[y];
+      bool hx = rx > seg_start[ux], hy = ry > seg_start[uy];
       if (!hx && !hy) return name_rank[ux] < name_rank[uy];
-      if (!hx) return false;  // X has arrival 0 => Y first
+      if (!hx) return false;  // X's run has arrival 0 => Y first
       if (!hy) return true;
-      // before(X,Y) = before(prev(Y), prev(X)): swap roles and step back
-      int nx = y - 1, ny = x - 1;
-      x = nx; y = ny;
+      // before(X,Y) = before(prev(run(Y)), prev(run(X))): swap roles and step back
+      x = ry - 1; y = rx - 1;
       dx = dru[x]; dy = dru[y];
     }
   }
 };
+
+// run_start for LessMerge: an inclusive max-scan of "p starts a run" (first slot of the user's segment,
+// or a dru different from the slot before; NaN never equals) over the user-sorted positions.  Tiles of
+// RS_TB, one short serial pass over the tile maxima, then the fix-up.
+constexpr int RS_TB = 1024;
+__global__ void __launch_bounds__(RS_TB) run_start_tiles(const double* __restrict__ dru_at, const int32_t* __restrict__ user_at,
+                                                          const int32_t* __restrict__ seg_start, int n,
+                                                          int32_t* __restrict__ run_start, int32_t* __restrict__ tile_max) {
+  __shared__ int wmax[RS_TB / 32];
+  const int p = blockIdx.x * RS_TB + threadIdx.x, lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  int v = 0;
+  if (p < n) v = (p == seg_start[user_at[p]] || !(dru_at[p - 1] == dru_at[p])) ? p : 0;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, v, o); if (lane >= o) v = max(v, y); }
+  if (lane == 31) wmax[w] = v;
+  __syncthreads();
+  if (w == 0) {
+    int t = wmax[lane];
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, t, o); if (lane >= o) t = max(t, y); }
+    wmax[lane] = t;
+  }
+  __syncthreads();
+  if (w) v = max(v, wmax[w - 1]);
+  if (p < n) run_start[p] = v;
+  if (threadIdx.x == RS_TB - 1) tile_max[blockIdx.x] = v;
+}
+__global__ void run_start_carry(int32_t* tile_max, int nb) {   // one thread: exclusive prefix max
+  int m = 0;
+  for (int b = 0; b < nb; b++) { const int t = tile_max[b]; tile_max[b] = m; m = max(m, t); }
+}
+__global__ void __launch_bounds__(RS_TB) run_start_fix(int32_t* run_start, const int32_t* tile_max, int n) {
+  const int p = blockIdx.x * RS_TB + threadIdx.x;
+  if (p < n) run_start[p] = max(run_start[p], tile_max[blockIdx.x]);
+}
 
 __global__ void scatter_dru_kernel(const int32_t* __restrict__ idx, const double* __restrict__ dru_at,
                                    int n, double* __restrict__ dru_task) {
@@ -591,6 +633,7 @@ extern "C" int32_t cook_rank(cook_pool* pool, const cook_tasks_soa* running,
   sz.add<int32_t>(N / QF_TB + 2); sz.add<GridFlag>(1);
   for (int k = 0; k < 3; k++) sz.add<double>(N + 1);     // order-wide scans: tile-local sums
   sz.add<double>(3 * (N / OS_TILE + 2)); sz.add<int32_t>(N + 1); sz.add<int32_t>(N / OS_TILE + 2);
+  sz.add<int32_t>(N + 1); sz.add<int32_t>(N / RS_TB + 2);  // run starts of equal dru, tile maxima
   CK(pool, ar.reserve(sz.off + 4096));
   ar.reset();
 
@@ -638,6 +681,8 @@ extern "C" int32_t cook_rank(cook_pool* pool, const cook_tasks_soa* running,
   double* d_os_pm = ar.take<double>(N + 1); double* d_os_pc = ar.take<double>(N + 1); double* d_os_pg = ar.take<double>(N + 1);
   double* d_os_b = ar.take<double>(3 * (os_nb + 1));
   int32_t* d_os_pv = ar.take<int32_t>(N + 1); int32_t* d_os_bv = ar.take<int32_t>(os_nb + 1);
+  const int rs_nb = (N + RS_TB - 1) / RS_TB;
+  int32_t* d_run_start = ar.take<int32_t>(N + 1); int32_t* d_rs_tile = ar.take<int32_t>(rs_nb + 1);
   if (ar.failed) return set_err(pool, COOK_E_OOM, "cook_rank: arena exhausted");
   CK(pool, cudaMemsetAsync(d_gf, 0, sizeof(GridFlag), st));
   CK(pool, cudaMemsetAsync(d_seg_start, 0, sizeof(int32_t) * U, st));
@@ -667,9 +712,12 @@ extern "C" int32_t cook_rank(cook_pool* pool, const cook_tasks_soa* running,
         d_idx, t, uc, d_seg_start, d_seg_end, U, pool->dru_mode, params->max_over_quota_jobs,
         d_dru_at, d_counters, d_gf, N);
   }
+  run_start_tiles<<<rs_nb, RS_TB, 0, st>>>(d_dru_at, d_user_at, d_seg_start, N, d_run_start, d_rs_tile);
+  run_start_carry<<<1, 1, 0, st>>>(d_rs_tile, rs_nb);
+  run_start_fix<<<rs_nb, RS_TB, 0, st>>>(d_run_start, d_rs_tile, N);
   iota_kernel<<<nb, TB, 0, st>>>(d_pos, N);
   CK(pool, csort::sort_indices(d_pos, d_tmp, N,
-                               LessMerge{d_dru_at, d_user_at, d_seg_start, d_name_rank}, st));
+                               LessMerge{d_dru_at, d_user_at, d_seg_start, d_name_rank, d_run_start}, st));
   QueueFilterArgs qa;
   qa.pos_sorted = d_pos; qa.idx = d_idx; qa.n_kept = d_counters; qa.R = R;
   qa.cpus = d_cpus; qa.mem = d_mem; qa.gpus = d_gpus;
@@ -718,7 +766,7 @@ extern "C" int32_t cook_rank(cook_pool* pool, const cook_tasks_soa* running,
     ps.d2h_bytes = (int64_t)n_out * 4 + (out_order ? (int64_t)n_kept * 4 : 0) + (out_dru ? (int64_t)N * 8 : 0) + 8;
     int nl = 0;
     for (long long w = csort::TILE; w < N; w <<= 1) nl += 2;   // the two sorts' merge passes
-    ps.n_launches = nl + 12;
+    ps.n_launches = nl + 15;
   }
   *out_n = n_out;
   if (out_order_n) *out_order_n = n_kept;
